@@ -7,6 +7,7 @@ observations), one process per GPU.
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...     # the reference's NumPy CPU step (oracle port)
+    python bench.py ... --dump-outputs DIR   # also save the last timed step's outputs (.npy)
 
 One "step" = one rollout timestep of every env replica on this rank:
 policy forward (2 policies) -> sample 2 action heads -> env.step -> bookkeeping ->
@@ -177,6 +178,37 @@ def build_engine(n_envs, seed, graph_steps, use_graph=True, forward_dtype=None,
                            use_pair_forward=pair_forward)
     engine.stats = stats
     return wrapper, engine, sampler, policy_map
+
+
+def last_step_outputs(engine):
+    """Host copies of what engine.rollout() hands its caller for the rollout's last timestep:
+    per policy the actions sampled and the rewards received in that step and the
+    observations it produced (the next step's policy input), and the done flags."""
+    T = engine.T
+    out = {"done_flags": engine._tensor("done_flags_batch")[T - 1]}
+    for p in engine.policies:
+        out[f"observations_{p}"] = engine.cur_obs[p]
+        out[f"actions_{p}"] = engine._tensor(f"sampled_actions_batch_{p}")[T - 1]
+        out[f"rewards_{p}"] = engine._tensor(f"rewards_batch_{p}")[T - 1]
+    return {k: v.float().cpu().numpy() for k, v in out.items()}
+
+
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def write_outputs(outputs, out_dir):
+    """One float32 .npy per array, DUMP_LIMIT_BYTES in all at most: beyond that, every
+    array keeps the same fixed, seeded sample of env replicas (axis 0)."""
+    n_envs = next(iter(outputs.values())).shape[0]
+    keep = np.arange(n_envs)
+    budget = DUMP_LIMIT_BYTES - 4096 * len(outputs)          # .npy headers
+    total = sum(a.nbytes for a in outputs.values())
+    if total > budget:
+        n = max(1, n_envs * budget // total)
+        keep = np.sort(np.random.RandomState(0).choice(n_envs, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a[keep], np.float32))
 
 
 def issue_roofline(kernel, kernel_ms, E, N):
@@ -522,7 +554,7 @@ def run_config3(args):
 
     for _ in range(max(3, math.ceil(W / T))):
         eng.rollout()
-    reps = args.reps if args.reps > 0 else 9
+    reps = max(1, args.reps)
     rep_ms = []
     with ClockSampler(local_rank) as clocks:
         c0 = wlib.launch_count()
@@ -806,7 +838,7 @@ def run_train_mode(args):
     T = args.train_steps
     n_iters = max(1, args.steps // T)
     K = n_iters * T
-    reps = args.reps if args.reps > 0 else 5
+    reps = max(1, args.reps)
     with ClockSampler(local_rank) as clocks:
         stats = train_iteration_stats(args, world, rank, local_rank, n_iters, reps,
                                       warm_iters=max(3, math.ceil(args.warmup / T)))
@@ -871,13 +903,20 @@ def main():
                          "measured slower, see scripts/ab_forward_modes.py")
     ap.add_argument("--copy-streams", type=int, default=4,
                     help="streams the e2e observation D2H copy is split over")
-    ap.add_argument("--reps", type=int, default=0,
-                    help="repetitions of the K-step timed region (median reported); 0 = auto")
+    ap.add_argument("--reps", type=int, default=1,
+                    help="repetitions of the K-step timed region (median reported)")
     ap.add_argument("--skip-ref-gpu", action="store_true",
                     help="do not time the reference's own CUDA kernels (oracle/_ref fatbin)")
     ap.add_argument("--cta-threads", type=int, default=0,
                     help="A/B switch: thread budget of one tag_continuous CTA (wdb_set_option)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the rollout's last timestep handed "
+                         "to its caller to DIR/<name>.npy (float32; at most 64 MB, a fixed "
+                         "seeded sample of env replicas beyond that)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.config == 3 or args.impl == "reference"
+                              or args.mode == "train"):
+        ap.error("--dump-outputs: only the b200 rollout of configs 2 and 4")
     if args.config == 3:
         return run_reference_arm_config3(args) if args.impl == "reference" else run_config3(args)
     _ACTIVE["config"] = args.config
@@ -947,10 +986,10 @@ def main():
 
     # ---- timed region: exactly K steps, CUDA events, barrier + synchronize on both sides.
     # A K-step region of a few milliseconds is at the mercy of one clock ramp or one slow
-    # replay, so the region is repeated `reps` times back to back (each repetition is
-    # exactly K steps with its own barrier / event pair / max over ranks) and the MEDIAN
-    # repetition is reported; all repetitions are listed in `ms_per_step_reps`.
-    reps = args.reps if args.reps > 0 else (1 if K >= 1000 else 5 if K >= 200 else 9)
+    # replay; --reps R repeats it R times back to back (each repetition is exactly K steps
+    # with its own barrier / event pair / max over ranks) and reports the MEDIAN repetition;
+    # all repetitions are listed in `ms_per_step_reps`.
+    reps = max(1, args.reps)
     engine.stats.zero_()
     rep_ms = []
     with ClockSampler(local_rank) as clocks:
@@ -969,6 +1008,7 @@ def main():
             rep_ms.append(float(t.item()))
         stats_timed = engine.stats.cpu().numpy().tolist()
         c1 = wlib.launch_count()
+        outputs = last_step_outputs(engine) if args.dump_outputs else None
         # the timed region lasts tens of milliseconds, one nvidia-smi poll at most: keep the
         # same rollout running (untimed) for ~0.4 s so that the clock samples are taken under
         # exactly this load
@@ -1156,6 +1196,8 @@ def main():
         except Exception as err:  # noqa: BLE001
             line["cpu_c_oracle"] = {"error": str(err)}
     print(json.dumps(line))
+    if outputs is not None:
+        write_outputs(outputs, args.dump_outputs)
     if world > 1:
         dist.destroy_process_group()
     return 0

@@ -1,5 +1,60 @@
 """Shared helpers for the parity tests (state construction from golden fixtures)."""
+import hashlib
+import os
+
 import numpy as np
+
+REF_KERNELS_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden",
+                                  "ref_kernels.npz")
+
+
+def fingerprint(a, bitwise=False):
+    """32-bit fingerprint of an array's bytes in C order (torch tensors are copied to the
+    host).  Equal arrays give equal fingerprints; a different array matches by chance with
+    probability 2**-32.  Unless `bitwise`, -0.0 counts as +0.0, as in torch.equal."""
+    if hasattr(a, "detach"):
+        a = a.detach().cpu().numpy()
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f" and not bitwise:
+        a = a + a.dtype.type(0)          # -0.0 + 0.0 == +0.0; every other value unchanged
+    digest = hashlib.blake2b(a.tobytes(), digest_size=4).digest()
+    return np.uint32(int.from_bytes(digest, "little"))
+
+
+def row_fingerprints(a, bitwise=False):
+    """fingerprint() of every row (leading index) of `a`."""
+    return np.array([fingerprint(r, bitwise) for r in a], np.uint32)
+
+
+class RefTrace:
+    """What the reference's own kernels computed in one parity case, step by step, as
+    fingerprints (tests/golden/ref_kernels.npz, written by
+    tests/golden/make_ref_kernel_golden.py).  The full outputs are too large to store, and
+    the comparisons against the reference are bit-exact, so a fingerprint is all they need.
+    Entry `<case>.<key>` holds one fingerprint per step, or one per row and step.
+    `bitwise`: as the case was recorded (see fingerprint())."""
+
+    _data = None
+
+    def __init__(self, case, bitwise=False):
+        if RefTrace._data is None:
+            RefTrace._data = dict(np.load(REF_KERNELS_GOLDEN, allow_pickle=False))
+        self.case, self.bitwise = case, bitwise
+        assert any(k.startswith(case + ".") for k in RefTrace._data), case
+
+    def _entry(self, key):
+        return RefTrace._data[f"{self.case}.{key}"]
+
+    def steps(self, key):
+        return len(self._entry(key))
+
+    def same(self, t, key, ours):
+        """`ours` equals the reference's `key` at step t."""
+        return fingerprint(ours, self.bitwise) == self._entry(key)[t]
+
+    def same_rows(self, t, key, ours):
+        """Per row of `ours`: equal to that row of the reference's `key` at step t."""
+        return row_fingerprints(ours, self.bitwise) == self._entry(key)[t]
 
 
 def tc_cfg_from_fixture(fx):

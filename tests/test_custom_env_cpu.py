@@ -46,19 +46,6 @@ def test_registrar_keeps_custom_source_paths():
         reg.add_cuda_env_src_path("Bad", "/tmp/not_cuda.py")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="build container only")
-@pytest.mark.parametrize("rel,kernel", [
-    ("example_envs/tag_gridworld/tag_gridworld_step_pycuda.cu", "CudaTagGridWorldStep"),
-    ("example_envs/tag_continuous/tag_continuous_step_pycuda.cu", "CudaTagContinuousStep"),
-    ("example_envs/dummy_env/test_step.cu", "testkernel")])
-def test_reference_env_files_compile_unchanged(rel, kernel, tmp_path, monkeypatch):
-    """The reference's own env sources are 'custom env files' in this sense: they must go
-    through the plug-in path as they are (read in place, nothing copied)."""
-    monkeypatch.setenv("WDB_KERNEL_CACHE", str(tmp_path))
-    cubin = ck.compile_module(os.path.join("/root/reference", rel), 4, 6, 1)
-    assert kernel in ck.kernel_names(cubin)
-
-
 def test_marshal_follows_pycuda_rules():
     import ctypes
 

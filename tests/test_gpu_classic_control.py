@@ -1,9 +1,9 @@
 """GPU parity of the single-agent classic-control steps (CartPole + SURVEY 8 row f2:
 MountainCar, ContinuousMountainCar, Pendulum, Acrobot), called through the C ABI, against
 
-(a) the REFERENCE's own numba kernels, compiled by numba from /root/reference in the build
-    container (oracle/build_ref_numba.py -> oracle/_ref/numba_*.cubin) and launched next to
-    ours on identical inputs (oracle/ref_numba.py), and
+(a) what the REFERENCE's own numba kernels (compiled by numba, oracle/build_ref_numba.py)
+    computed from identical inputs, stored as per-step fingerprints
+    (tests/golden/ref_kernels.npz, tests/helpers.py RefTrace), and
 (b) the C oracle (oracle/wd_oracle.c, glibc libm on the host).
 
 Every step is an independent single-step comparison on freshly drawn states that cover the
@@ -11,11 +11,9 @@ clipping / wrapping / terminal branches (teacher forcing: the integrators are ch
 free-running comparison would only measure that).
 
 Bars (written here, cited in DESIGN.md):
-  * vs the reference numba binaries: float32 state / obs / reward within 1e-6 abs-or-rel
-    (the only freedom is where ptxas fuses float64 multiply-adds before the float32 store);
-    the bit-identical fraction is measured, reported and held to MIN_BIT_IDENTICAL; done /
-    timestep flags must be IDENTICAL for every env whose float outputs are bit-identical (a
-    last-bit difference may legitimately flip a threshold test).
+  * vs the reference numba binaries: float32 state / obs / reward, done and timestep
+    BIT-identical for every env-step, as measured on the B200
+    (profiles/r3_classic_control_parity.json).
   * vs the C oracle: within 1e-5 abs-or-rel (Acrobot 2e-4; libm vs libdevice), flags equal except for at
     most MAX_BRANCH_FLIPS threshold flips.
 A JSON summary goes to gpurun_out/classic_control_parity.json.
@@ -27,7 +25,7 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import ref_numba
+from helpers import RefTrace
 
 pytestmark = pytest.mark.gpu
 
@@ -48,12 +46,6 @@ ORACLE_TOL = {"acrobot": 2e-4}
 # same ulps come out at 1e-3.  The reference numba binary is compared on ALL rows.
 ORACLE_ROWS = {"acrobot": lambda s0: (np.abs(s0[:, 0, 2]) <= PI) & (np.abs(s0[:, 0, 3]) <= 2 * PI)}
 PI = np.pi
-
-# Fraction of env-steps whose float32 outputs must be BIT-identical to the reference numba
-# binary (seeded, deterministic inputs): all of them, as measured on the B200
-# (profiles/r3_classic_control_parity.json).
-MIN_BIT_IDENTICAL = {"cartpole": 1.0, "mountain_car": 1.0, "continuous_mountain_car": 1.0,
-                     "pendulum": 1.0, "acrobot": 1.0}
 
 _CARTPOLE_CONSTS = [9.8, 0.1, 1.1, 0.5, 0.05, 10.0, 0.02, 12 * 2 * np.pi / 360, 2.4]
 _MC_CONSTS = [-1.2, 0.6, 0.07, 0.5, 0.0, 0.001, 0.0025]
@@ -111,21 +103,17 @@ def test_step_vs_reference_numba_and_oracle(name, wdb_lib, oracle_lib):
     sdim, odim, adtype, consts, draw_state, draw_action = ENVS[name]
     ours = getattr(wdb_lib, f"wdb_{name}_step")
     oracle_fn = getattr(oracle_lib, f"wd_oracle_{name}_step")
-    if not ref_numba.available(name):
-        pytest.fail(f"oracle/_ref/numba_{name}.cubin missing (python oracle/build_ref_numba.py)")
-    ref = ref_numba.RefNumbaKernel(name)
+    ref = RefTrace(f"cc_{name}", bitwise=True)
     rs = np.random.RandomState(20260923 + len(name))
     p = wlib.ptr
     cuda = lambda a: torch.from_numpy(np.ascontiguousarray(a)).cuda()  # noqa: E731
 
     n_samples = 0
-    bit_equal = 0
-    max_abs_ref = 0.0
     max_abs_oracle = 0.0
     flag_flips_oracle = 0
-    bad_ref = bad_oracle = 0
+    bad_oracle = 0
     done_seen = set()
-    for _ in range(STEPS):
+    for t in range(STEPS):
         s0 = draw_state(rs, E).astype(np.float32).reshape(E, 1, sdim)
         act = draw_action(rs, E).astype(adtype).reshape(E, 1, 1)
         ts0 = rs.randint(0, EP_LEN, E).astype(np.int32)
@@ -137,12 +125,6 @@ def test_step_vs_reference_numba_and_oracle(name, wdb_lib, oracle_lib):
         d_obs = torch.full((E, 1, odim), 7.0, device="cuda")
         wlib.check(ours(wlib.stream_ptr(), E, p(d_s), p(d_a), p(d_done), p(d_rew), p(d_obs),
                         *consts, p(d_ts), EP_LEN))
-        # the reference's numba kernel (same argument order, no n_envs)
-        r_s, r_ts = cuda(s0), cuda(ts0)
-        r_done = torch.zeros(E, dtype=torch.int32, device="cuda")
-        r_rew = torch.full((E, 1), 7.0, device="cuda")
-        r_obs = torch.full((E, 1, odim), 7.0, device="cuda")
-        ref(E, r_s, d_a, r_done, r_rew, r_obs, *consts, r_ts, EP_LEN)
         torch.cuda.synchronize()
         # C oracle
         h_s, h_ts = s0.copy(), ts0.copy()
@@ -153,23 +135,16 @@ def test_step_vs_reference_numba_and_oracle(name, wdb_lib, oracle_lib):
 
         mine = np.concatenate([d_s.cpu().numpy().reshape(E, -1), d_obs.cpu().numpy().reshape(E, -1),
                                d_rew.cpu().numpy()], 1)
-        theirs = np.concatenate([r_s.cpu().numpy().reshape(E, -1),
-                                 r_obs.cpu().numpy().reshape(E, -1), r_rew.cpu().numpy()], 1)
         host = np.concatenate([h_s.reshape(E, -1), h_obs.reshape(E, -1), h_rew], 1)
-        assert np.isfinite(mine).all() and np.isfinite(theirs).all()
+        assert np.isfinite(mine).all()
 
         # ---- (a) vs the reference numba binary
-        ok = _close(mine, theirs, 1e-6).all(1)
-        bad_ref += int((~ok).sum())
-        assert bad_ref <= MAX_BRANCH_FLIPS, (name, "vs reference numba", mine[~ok][:3], theirs[~ok][:3])
-        same_bits = (mine.view(np.uint32) == theirs.view(np.uint32)).all(1)
-        bit_equal += int(same_bits.sum())
+        assert ref.same(t, "outputs", mine), (name, t, "state / obs / reward vs reference numba")
+        m_done = d_done.cpu().numpy()
+        assert ref.same(t, "done", m_done), (name, t, "done vs reference numba")
+        assert ref.same(t, "timestep", d_ts), (name, t, "timestep vs reference numba")
         n_samples += E
-        max_abs_ref = max(max_abs_ref, float(np.abs(mine - theirs)[ok].max()))
-        m_done, t_done = d_done.cpu().numpy(), r_done.cpu().numpy()
-        assert (m_done[same_bits] == t_done[same_bits]).all(), (name, "done vs reference numba")
-        assert torch.equal(d_ts, r_ts)
-        done_seen |= set(np.unique(t_done).tolist())
+        done_seen |= set(np.unique(m_done).tolist())
 
         # ---- (b) vs the C oracle
         ok = _close(mine, host, ORACLE_TOL.get(name, 1e-5)).all(1)
@@ -184,18 +159,14 @@ def test_step_vs_reference_numba_and_oracle(name, wdb_lib, oracle_lib):
         flag_flips_oracle += int(((m_done != h_done) & ok).sum())
         assert (d_ts.cpu().numpy() == h_ts).all()
 
-    frac = bit_equal / n_samples
-    _report(name, {"env_steps": n_samples, "bit_identical_vs_reference_numba": frac,
-                   "rows_on_other_branch_vs_reference_numba": bad_ref,
+    _report(name, {"env_steps": n_samples, "bit_identical_vs_reference_numba": 1.0,
                    "rows_on_other_branch_vs_c_oracle": bad_oracle,
-                   "max_abs_diff_vs_reference_numba": max_abs_ref,
                    "max_abs_diff_vs_c_oracle": max_abs_oracle,
                    "done_flag_flips_vs_c_oracle": flag_flips_oracle,
                    "done_values_seen": sorted(int(v) for v in done_seen)})
-    print(f"[classic-control parity] {name}: {frac:.6f} of {n_samples} env-steps bit-identical "
-          f"to the reference numba binary, max |diff| {max_abs_ref:.3g}; vs C oracle max |diff| "
-          f"{max_abs_oracle:.3g}, {flag_flips_oracle} done flips")
-    assert frac >= MIN_BIT_IDENTICAL[name], (name, frac)
+    print(f"[classic-control parity] {name}: all {n_samples} env-steps bit-identical to the "
+          f"reference numba binary; vs C oracle max |diff| {max_abs_oracle:.3g}, "
+          f"{flag_flips_oracle} done flips")
     assert flag_flips_oracle <= MAX_BRANCH_FLIPS, (name, flag_flips_oracle)
     assert 1 in done_seen                       # the episode-end branch ran
     if name == "mountain_car":

@@ -1,6 +1,6 @@
 """GPU parity tests of the env step kernels, called through the C ABI exactly like the
-managers do, against (a) the CPU oracle and (b) the reference's own CUDA kernels
-(oracle/_ref/*.fatbin) on identical inputs.
+managers do, against (a) the CPU oracle and (b) what the reference's own CUDA kernels
+computed from identical inputs (fingerprints in tests/golden/ref_kernels.npz).
 
 Bars: integer / index / flag outputs bit-exact; float32 outputs within 1e-5 abs-or-rel
 against the CPU oracle (libm vs libdevice sin/cos differ in the last bit) and BIT-EXACT
@@ -11,7 +11,7 @@ import torch
 
 import oracle
 from conftest import load_golden
-from helpers import close, copy_state, tc_cfg_from_fixture, tc_state_from_fixture
+from helpers import RefTrace, close, copy_state, tc_cfg_from_fixture, tc_state_from_fixture
 
 pytestmark = pytest.mark.gpu
 
@@ -122,15 +122,12 @@ def test_tag_continuous_teacher_forced_vs_oracle(wdb_lib, name, tc_history):
 @pytest.mark.parametrize("shape", [(2, 5), (4, 23), (8, 105)])
 @pytest.mark.parametrize("full_obs", [False, True])
 def test_tag_continuous_bit_exact_vs_reference_cuda(wdb_lib, shape, full_obs, tc_history):
-    """Free-running rollouts of OUR kernel and the REFERENCE kernel from the same
-    initial state with the same actions; every output array must be bit-identical.
-    (Steps where one tagger is credited for >= 2 tags are where the reference has a data
-    race -- tag_continuous_step_pycuda.cu:324-329 -- and are excluded for rewards.)"""
-    from oracle import ref_cuda
-
+    """Free-running rollout of OUR kernel against what the REFERENCE kernel computed from
+    the same initial state with the same actions (RefTrace); every output array must be
+    bit-identical.  (Steps where one tagger is credited for >= 2 tags are where the
+    reference has a data race -- tag_continuous_step_pycuda.cu:324-329 -- and are excluded
+    for rewards.)"""
     E, N = shape
-    if not ref_cuda.available(E, N, 1):
-        pytest.skip("reference fatbin for this shape was not shipped")
     fxname = {5: "test3", 23: "partial_mid", 105: "config2_short"}[N]
     fx = load_golden(f"tag_continuous_numpy_{fxname}.npz")
     cfg = tc_cfg_from_fixture(fx)
@@ -143,51 +140,42 @@ def test_tag_continuous_bit_exact_vs_reference_cuda(wdb_lib, shape, full_obs, tc
     K = int(cfg["num_other_agents_observed"])
     st0["nearest_neighbor_ids"] = np.zeros((E, N, K), np.int32)
     F = _obs_dim(cfg, N)
-    ref = ref_cuda.RefModule(E, N, 1)
-    a_st, b_st, dcfg = _dev(st0), _dev(st0), _dev(cfg)
-    a_obs, b_obs = torch.zeros((E, N, F), device="cuda"), torch.zeros((E, N, F), device="cuda")
-    a_rew, b_rew = torch.zeros((E, N), device="cuda"), torch.zeros((E, N), device="cuda")
-    nd = torch.zeros((E, N, N - 1), device="cuda")
-    nid = torch.zeros((E, N, N - 1), dtype=torch.int32, device="cuda")
+    ref = RefTrace(f"tc_E{E}_N{N}_full{int(full_obs)}")
+    a_st, dcfg = _dev(st0), _dev(cfg)
+    a_obs = torch.zeros((E, N, F), device="cuda")
+    a_rew = torch.zeros((E, N), device="cuda")
     init = _dev(st0)
     rs = np.random.RandomState(7)
     racy_steps = 0
     for t in range(150):
         done = a_st["_done_"].cpu().numpy()
         for e in np.nonzero(done)[0]:
-            for st in (a_st, b_st):
-                for k in st:
-                    st[k][e] = init[k][e]
+            for k in a_st:
+                a_st[k][e] = init[k][e]
         actions = torch.from_numpy(_random_actions(rs, E, N, cfg)).cuda()
         alive_before = a_st["still_in_the_game"].clone()
         wdb_tc_step(wdb_lib, a_st, dcfg, actions, a_obs, a_rew)
-        ref.tag_continuous_step(b_st, dcfg, actions, b_obs, b_rew, nd, nid)
         torch.cuda.synchronize()
         for k in STATE_F + STATE_I:
             if k == "num_runners":
                 continue  # racy decrement in the reference; checked via alive flags
-            assert torch.equal(a_st[k], b_st[k]), (t, k)
-        assert torch.equal(a_obs, b_obs), (t, "obs", (a_obs != b_obs).nonzero()[:4])
+            assert ref.same(t, k, a_st[k]), (t, k)
+        assert ref.same(t, "obs", a_obs), (t, "obs")
         if not full_obs:
             valid = torch.clamp(alive_before.sum(1, keepdim=True) - alive_before, max=K)
             mask = (torch.arange(K, device="cuda")[None, None] < valid[:, :, None]) & \
                    (alive_before[:, :, None] > 0)
-            assert torch.equal(a_st["nearest_neighbor_ids"][mask],
-                               b_st["nearest_neighbor_ids"][mask]), t
-        tagged = (alive_before - a_st["still_in_the_game"]).sum(1) if \
+            assert ref.same(t, "nearest_neighbor_ids", a_st["nearest_neighbor_ids"][mask]), t
+        tagged = (alive_before - a_st["still_in_the_game"]).sum(1).cpu().numpy() if \
             int(cfg["runner_exits_game_after_tagged"]) else None
-        same = (a_rew == b_rew).all(1)
-        if not bool(same.all()):
+        same = ref.same_rows(t, "rewards", a_rew)
+        if not same.all():
             # only envs with >= 2 simultaneous tags may differ (reference race)
-            bad = (~same).nonzero().reshape(-1)
+            bad = np.nonzero(~same)[0]
             assert tagged is not None and bool((tagged[bad] >= 2).all()), (t, bad)
             racy_steps += 1
-            b_st["num_runners"].copy_(a_st["num_runners"])
-            b_st["_done_"].copy_(a_st["_done_"])
         else:
-            assert torch.equal(a_st["num_runners"], b_st["num_runners"]) or tagged is not None
-            b_st["num_runners"].copy_(a_st["num_runners"])
-            b_st["_done_"].copy_(a_st["_done_"])
+            assert ref.same(t, "num_runners", a_st["num_runners"]) or tagged is not None
     assert racy_steps < 40
 
 
@@ -348,12 +336,8 @@ def test_gridworld_bit_exact_vs_oracle(wdb_lib, oracle_lib, N, B, full):
 
 @pytest.mark.parametrize("full", [True, False])
 def test_gridworld_bit_exact_vs_reference_cuda(wdb_lib, full):
-    from oracle import ref_cuda
-
     E, N, B, T = 2, 5, 4, 20
-    if not ref_cuda.available(E, N, 1):
-        pytest.skip("reference fatbin not shipped")
-    ref = ref_cuda.RefModule(E, N, 1)
+    ref = RefTrace(f"gw_full{int(full)}")
     cfg = dict(wall_hit_penalty=0.1, tag_reward_for_tagger=10.0, tag_penalty_for_runner=2.0,
                step_cost_for_tagger=0.01, use_full_observation=full, world_boundary=B)
     F = 4 * N + 1 if full else 6
@@ -364,20 +348,16 @@ def test_gridworld_bit_exact_vs_reference_cuda(wdb_lib, full):
     A = dict(x=x0.clone(), y=y0.clone(), done=torch.zeros(E, dtype=torch.int32, device="cuda"),
              ts=torch.zeros(E, dtype=torch.int32, device="cuda"),
              rew=torch.zeros((E, N), device="cuda"), obs=torch.zeros((E, N, F), device="cuda"))
-    Bs = {k: v.clone() for k, v in A.items()}
     for t in range(100):
-        for S in (A, Bs):
-            d = S["done"] > 0
-            S["x"][d], S["y"][d] = x0[d], y0[d]
-            S["ts"][d], S["done"][d] = 0, 0
+        d = A["done"] > 0
+        A["x"][d], A["y"][d] = x0[d], y0[d]
+        A["ts"][d], A["done"][d] = 0, 0
         actions = torch.from_numpy(rs.randint(0, 5, (E, N)).astype(np.int32)).cuda()
         wdb_gw_step(wdb_lib, A["x"], A["y"], actions, A["done"], A["rew"], A["obs"], cfg,
                     full, B, A["ts"], T, moves)
-        ref.tag_gridworld_step(Bs["x"], Bs["y"], actions, Bs["done"], Bs["rew"], Bs["obs"],
-                               cfg, Bs["ts"], T, MOVES)
         torch.cuda.synchronize()
         for k in A:
-            assert torch.equal(A[k], Bs[k]), (t, k)
+            assert ref.same(t, k, A[k]), (t, k)
 
 
 # ------------------------------------------------------------------ cartpole
@@ -517,46 +497,34 @@ def test_tag_continuous_large_agent_counts_vs_oracle(wdb_lib, N, n_taggers, E, g
 @pytest.mark.parametrize("N,n_taggers,E,grid", [(330, 20, 3, 30.0)])
 def test_tag_continuous_large_agent_counts_vs_reference_cuda(wdb_lib, N, n_taggers, E, grid,
                                                              tc_history):
-    """The same large configurations against the REFERENCE's own kernel (compiled in place,
-    oracle/build_ref.py): state, observations and neighbour ids bit-identical, including the
-    order of neighbours whose float distances tie exactly."""
-    from oracle import ref_cuda
-
-    if not ref_cuda.available(E, N, 1):
-        pytest.skip("reference fatbin for this shape was not shipped")
-    if N > 512:
-        pytest.skip("the reference kernel cannot be launched with 1024 threads per block on "
-                    "sm_100a (CUDA_ERROR_LAUNCH_OUT_OF_RESOURCES: its register use); config-4 "
-                    "sizes are checked against the C oracle only")
+    """The same large configurations against what the REFERENCE's own kernel computed
+    (RefTrace): state, observations and neighbour ids bit-identical, including the order of
+    neighbours whose float distances tie exactly.  (The reference kernel cannot be launched
+    with 1024 threads per block on sm_100a -- CUDA_ERROR_LAUNCH_OUT_OF_RESOURCES, its
+    register use -- so config-4 sizes are checked against the C oracle above and against
+    the reference's multi-block mode in tests/test_gpu_wide.py.)"""
     K = 10
     cfg, st0 = _tc_synthetic(N, n_taggers, K, E, grid, seed=N)
     F = 7 * K + 1
-    ref = ref_cuda.RefModule(E, N, 1)
-    a_st, b_st, dcfg = _dev(st0), _dev(st0), _dev(cfg)
-    a_obs, b_obs = torch.zeros((E, N, F), device="cuda"), torch.zeros((E, N, F), device="cuda")
-    a_rew, b_rew = torch.zeros((E, N), device="cuda"), torch.zeros((E, N), device="cuda")
-    nd = torch.zeros((E, N, N - 1), device="cuda")
-    nid = torch.zeros((E, N, N - 1), dtype=torch.int32, device="cuda")
-    nd2, nid2 = torch.zeros_like(nd), torch.zeros_like(nid)
+    ref = RefTrace(f"tc_large_E{E}_N{N}")
+    a_st, dcfg = _dev(st0), _dev(cfg)
+    a_obs = torch.zeros((E, N, F), device="cuda")
+    a_rew = torch.zeros((E, N), device="cuda")
+    nd2 = torch.zeros((E, N, N - 1), device="cuda")
+    nid2 = torch.zeros((E, N, N - 1), dtype=torch.int32, device="cuda")
     rs = np.random.RandomState(1)
     for t in range(10):
         actions = torch.from_numpy(_random_actions(rs, E, N, cfg)).cuda()
         alive_before = a_st["still_in_the_game"].clone()
         wdb_tc_step(wdb_lib, a_st, dcfg, actions, a_obs, a_rew, nd2, nid2)
-        ref.tag_continuous_step(b_st, dcfg, actions, b_obs, b_rew, nd, nid)
         torch.cuda.synchronize()
         for k in STATE_F + ("still_in_the_game", "_timestep_"):
-            assert torch.equal(a_st[k], b_st[k]), (t, k)
+            assert ref.same(t, k, a_st[k]), (t, k)
         valid = torch.clamp(alive_before.sum(1, keepdim=True) - alive_before, max=K)
         mask = (torch.arange(K, device="cuda")[None, None] < valid[:, :, None]) & \
                (alive_before[:, :, None] > 0)
-        bad = ((a_st["nearest_neighbor_ids"] != b_st["nearest_neighbor_ids"]) & mask).nonzero()
-        assert len(bad) == 0, (t, bad[:6].tolist())
-        assert torch.equal(a_obs, b_obs), (t, "obs")
-        # the reference's racy tag bookkeeping: keep both trajectories on ours
-        b_st["num_runners"].copy_(a_st["num_runners"])
-        b_st["_done_"].copy_(a_st["_done_"])
-
+        assert ref.same(t, "nearest_neighbor_ids", a_st["nearest_neighbor_ids"][mask]), t
+        assert ref.same(t, "obs", a_obs), (t, "obs")
 
 
 @pytest.mark.parametrize("shape", [(4, 23), (8, 105)])

@@ -76,7 +76,7 @@ def _worker(rank, world, port, out):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 def test_flat_gradient_allreduce_and_two_rank_training_nccl():
     world, port = 2, _free_port()
     ctx = mp.get_context("spawn")

@@ -7,10 +7,10 @@ Three layers:
   * every parity test of tests/test_gpu_envs.py and the fused-step tests of
     tests/test_gpu_rollout.py re-run with blocks_per_env = 2 / 3 (the cluster kernel works at
     any env size), in all three k-nearest modes and with the x-window on and off;
-  * 1024 agents per env against the C oracle AND against the REFERENCE's own kernel compiled
-    with wkBlocksPerEnv = 2 and 4 (oracle/_ref/ref_E2_N1024_B{2,4}.fatbin: 512 / 256 threads
-    per block, which sm_100a can launch): state, observations, neighbour ids bit-identical,
-    no tie escape;
+  * 1024 agents per env against the C oracle AND against what the REFERENCE's own kernel
+    computed with wkBlocksPerEnv = 2 and 4 (512 / 256 threads per block, which sm_100a can
+    launch; fingerprints in tests/golden/ref_kernels.npz): state, observations, neighbour
+    ids bit-identical, no tie escape;
   * the reference's own multi-block test shape (2 envs x 5 agents x 2 blocks).
 """
 import numpy as np
@@ -19,6 +19,7 @@ import torch
 
 import test_gpu_envs as base
 import test_gpu_rollout as roll
+from helpers import RefTrace
 from test_gpu_envs import tc_history  # noqa: F401  (fixture: history / network / exact)
 
 pytestmark = pytest.mark.gpu
@@ -82,24 +83,19 @@ def test_wide_1024_agents_vs_oracle(wdb_lib, blocks, tc_history, window):  # noq
 @pytest.mark.parametrize("grid", [64.0, 20.0])
 @pytest.mark.parametrize("blocks", [2, 4])
 def test_wide_1024_agents_bit_exact_vs_reference_multiblock(wdb_lib, blocks, tc_history, grid):  # noqa: F811
-    """BASELINE config 4 size against the REFERENCE kernel in its own multi-block mode
-    (wkBlocksPerEnv = 2 / 4): bit-equality of state, observations and neighbour ids over a
-    free-running rollout -- no rank-wise tie escape.  grid = 20: ten times config 4's agent
-    density, so the candidate list of the threshold scan overflows all the time and the
-    window-limited network path (stats[3]) carries the selection."""
-    from oracle import ref_cuda
-
+    """BASELINE config 4 size against what the REFERENCE kernel computed in its own
+    multi-block mode (wkBlocksPerEnv = 2 / 4; RefTrace): bit-equality of state,
+    observations and neighbour ids over a free-running rollout -- no rank-wise tie escape.
+    grid = 20: ten times config 4's agent density, so the candidate list of the threshold
+    scan overflows all the time and the window-limited network path (stats[3]) carries the
+    selection."""
     E, N, K, n_taggers = 2, 1024, 10, 24
-    if not ref_cuda.available(E, N, blocks):
-        pytest.fail(f"oracle/_ref/ref_E{E}_N{N}_B{blocks}.fatbin was not shipped")
     cfg, st0 = base._tc_synthetic(N, n_taggers, K, E, grid, seed=N)
     F = 7 * K + 1
-    ref = ref_cuda.RefModule(E, N, blocks)
-    a_st, b_st, dcfg = base._dev(st0), base._dev(st0), base._dev(cfg)
-    a_obs, b_obs = torch.zeros((E, N, F), device="cuda"), torch.zeros((E, N, F), device="cuda")
-    a_rew, b_rew = torch.zeros((E, N), device="cuda"), torch.zeros((E, N), device="cuda")
-    nd = torch.zeros((E, N, N - 1), device="cuda")
-    nid = torch.zeros((E, N, N - 1), dtype=torch.int32, device="cuda")
+    ref = RefTrace(f"tc_wide_N{N}_B{blocks}_grid{int(grid)}")
+    a_st, dcfg = base._dev(st0), base._dev(cfg)
+    a_obs = torch.zeros((E, N, F), device="cuda")
+    a_rew = torch.zeros((E, N), device="cuda")
     rs = np.random.RandomState(1)
     stats = torch.zeros(4, dtype=torch.int32, device="cuda")
     base._BPE = blocks
@@ -109,24 +105,19 @@ def test_wide_1024_agents_bit_exact_vs_reference_multiblock(wdb_lib, blocks, tc_
             actions = torch.from_numpy(base._random_actions(rs, E, N, cfg)).cuda()
             alive_before = a_st["still_in_the_game"].clone()
             base.wdb_tc_step(wdb_lib, a_st, dcfg, actions, a_obs, a_rew, stats=stats)
-            ref.tag_continuous_step(b_st, dcfg, actions, b_obs, b_rew, nd, nid)
             torch.cuda.synchronize()
             for k in base.STATE_F + ("still_in_the_game", "_timestep_"):
-                assert torch.equal(a_st[k], b_st[k]), (t, k)
+                assert ref.same(t, k, a_st[k]), (t, k)
             valid = torch.clamp(alive_before.sum(1, keepdim=True) - alive_before, max=K)
             mask = (torch.arange(K, device="cuda")[None, None] < valid[:, :, None]) & \
                    (alive_before[:, :, None] > 0)
-            bad = ((a_st["nearest_neighbor_ids"] != b_st["nearest_neighbor_ids"]) & mask).nonzero()
-            assert len(bad) == 0, (t, bad[:6].tolist())
-            assert torch.equal(a_obs, b_obs), (t, "obs")
+            assert ref.same(t, "nearest_neighbor_ids", a_st["nearest_neighbor_ids"][mask]), t
+            assert ref.same(t, "obs", a_obs), (t, "obs")
             # rewards: identical except where the reference's racy `rewards[tagger] += ...`
             # may lose a credit (taggers only)
             is_runner = dcfg["agent_types"] == 0
-            assert torch.equal(a_rew[:, is_runner], b_rew[:, is_runner]), (t, "runner rewards")
+            assert ref.same(t, "runner_rewards", a_rew[:, is_runner]), (t, "runner rewards")
             tags += int((alive_before - a_st["still_in_the_game"]).sum())
-            # the reference's racy counters: keep both trajectories on ours
-            b_st["num_runners"].copy_(a_st["num_runners"])
-            b_st["_done_"].copy_(a_st["_done_"])
         assert tags > 0
         if tc_history and grid < 64.0:
             assert int(stats[3]) > 0, "the window-limited network path never ran"
@@ -139,37 +130,32 @@ def test_wide_reference_multiblock_shape(wdb_lib, tc_history):  # noqa: F811
     agents x 2 blocks per env), both kernels in multi-block mode."""
     from conftest import load_golden
     from helpers import tc_cfg_from_fixture, tc_state_from_fixture
-    from oracle import ref_cuda
 
     E, N, blocks = 2, 5, 2
-    if not ref_cuda.available(E, N, blocks):
-        pytest.fail("oracle/_ref/ref_E2_N5_B2.fatbin was not shipped")
     fx = load_golden("tag_continuous_numpy_test1.npz")
     cfg = tc_cfg_from_fixture(fx)
     st0 = tc_state_from_fixture(fx, E)
     assert st0["loc_x"].shape[1] == N
     F = base._obs_dim(cfg, N)
-    ref = ref_cuda.RefModule(E, N, blocks)
-    a_st, b_st, dcfg = base._dev(st0), base._dev(st0), base._dev(cfg)
-    a_obs, b_obs = torch.zeros((E, N, F), device="cuda"), torch.zeros((E, N, F), device="cuda")
-    a_rew, b_rew = torch.zeros((E, N), device="cuda"), torch.zeros((E, N), device="cuda")
-    nd = torch.zeros((E, N, N - 1), device="cuda")
-    nid = torch.zeros((E, N, N - 1), dtype=torch.int32, device="cuda")
+    ref = RefTrace(f"tc_multiblock_E{E}_N{N}_B{blocks}")
+    a_st, dcfg = base._dev(st0), base._dev(cfg)
+    a_obs = torch.zeros((E, N, F), device="cuda")
+    a_rew = torch.zeros((E, N), device="cuda")
     rs = np.random.RandomState(7)
     base._BPE = blocks
     try:
+        steps = 0
         for t in range(int(cfg["episode_length"]) - 1):
             if bool(a_st["_done_"].any()):
                 break
             actions = torch.from_numpy(base._random_actions(rs, E, N, cfg)).cuda()
             base.wdb_tc_step(wdb_lib, a_st, dcfg, actions, a_obs, a_rew)
-            ref.tag_continuous_step(b_st, dcfg, actions, b_obs, b_rew, nd, nid)
             torch.cuda.synchronize()
             for k in base.STATE_F + ("still_in_the_game", "_timestep_"):
-                assert torch.equal(a_st[k], b_st[k]), (t, k)
-            assert torch.equal(a_obs, b_obs), (t, "obs")
-            b_st["num_runners"].copy_(a_st["num_runners"])
-            b_st["_done_"].copy_(a_st["_done_"])
+                assert ref.same(t, k, a_st[k]), (t, k)
+            assert ref.same(t, "obs", a_obs), (t, "obs")
+            steps += 1
+        assert steps == ref.steps("obs")    # the reference's episode ended at the same step
     finally:
         base._BPE = 1
 

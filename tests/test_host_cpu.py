@@ -387,30 +387,29 @@ def test_param_scheduler_and_config_merge():
 
 def test_all_nine_reference_run_configs_are_present():
     """Every run config of warp_drive/training/run_configs/ has a twin here with the same
-    schema; where /root/reference is present (build container) the values are compared too
-    (saving.basedir, a path on the reference authors' machine, excepted)."""
-    import yaml
+    schema and the same values (saving.basedir, a path on the reference authors' machine,
+    excepted), compared through the fingerprints in tests/golden/reference_run_configs.json."""
+    import hashlib
+    import json
 
     from warp_drive_b200.training.trainer import load_run_config
 
+    with open(os.path.join(ROOT, "tests", "golden", "reference_run_configs.json")) as fp:
+        theirs = json.load(fp)["sha256"]
     names = ["default_configs", "single_acrobot", "single_cartpole",
              "single_continuous_mountain_car", "single_mountain_car", "single_pendulum",
              "tag_continuous", "tag_gridworld", "tag_gridworld_with_reset_pool"]
-    ref_dir = "/root/reference/warp_drive/training/run_configs"
+    assert set(theirs) == set(names) - {"default_configs"}
     for name in names:
         ours = load_run_config(name)
-        if name != "default_configs":
-            assert {"name", "env", "trainer", "policy", "saving"} <= set(ours)
-            for pol in ours["policy"].values():
-                assert pol["algorithm"] in ("A2C", "PPO", "DDPG")
-        path = os.path.join(ref_dir, f"{name}.yaml")
-        if name == "default_configs" or not os.path.exists(path):
+        if name == "default_configs":
             continue
-        with open(path, encoding="utf8") as fp:
-            theirs = yaml.safe_load(fp)
-        for cfg in (ours, theirs):
-            cfg["saving"].pop("basedir", None)
-        assert ours == theirs, name
+        assert {"name", "env", "trainer", "policy", "saving"} <= set(ours)
+        for pol in ours["policy"].values():
+            assert pol["algorithm"] in ("A2C", "PPO", "DDPG")
+        ours["saving"].pop("basedir", None)
+        text = json.dumps(ours, sort_keys=True).encode()
+        assert hashlib.sha256(text).hexdigest() == theirs[name], name
     ddpg = load_run_config("single_pendulum")
     assert ddpg["trainer"]["n_step"] == 5 and ddpg["policy"]["shared"]["tau"] == 0.05
     assert ddpg["policy"]["shared"]["model"]["actor"]["output_w"] == 2.0
